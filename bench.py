@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- generator-forward throughput of the CIPS-3D hot path on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): generator fwd images/sec @ FFHQ r256, 24 samples/ray.  A step is one
@@ -39,6 +39,8 @@ G_KWARGS = dict(fov=12, ray_start=0.88, ray_end=1.12, num_steps=12, h_stddev=0.3
                 hierarchical_sample=True, psi=1., sample_dist="gaussian")
 WEIGHT_SEED = 1234          # ffhq_exp.yaml:146; both arms: the (reference-identical) constructor init under this seed
 REF_ROOT = os.path.join(ROOT, "baseline", "_ref")
+DRAW_SEED = 2000            # the forward's random draws (jitter, camera, noise) in the timed steps: the same on every run
+DUMP_BYTES = 64 << 20       # --dump-outputs writes at most this much
 
 
 def bench_config(res, B, world):
@@ -62,6 +64,19 @@ def reference_generator(device):
     import ref_shim
     torch.manual_seed(WEIGHT_SEED)
     return ref_shim.build_reference_generator(device).to(device).eval()     # the constructor's `device` is only an attribute
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as <out_dir>/<name>.npy in float32.  One larger than its share of DUMP_BYTES is replaced by a
+    fixed seeded sample of its elements (the same positions for the same shape), so that two builds compare element
+    for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def peaks():
@@ -231,6 +246,8 @@ def main():
     ap.add_argument("--u8", action="store_true", help="also time the uint8-delivery end-to-end leg (c3d_image_to_u8: opt-in until that "
                     "kernel has passed its GPU tests on hardware -- a fault there must not cost the contract line)")
     ap.add_argument("--no-eager", action="store_true", help="skip the eager-torch-on-the-same-GPU comparison")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (the images and pitch/yaw "
+                    "of GeneratorNerfINR.forward) as DIR/<name>.npy, float32")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -265,8 +282,7 @@ def main():
 
     def step_resident():
         with torch.no_grad():
-            img, _ = G(zs_dev, img_size=res, nerf_noise=0.0, **kw)
-        return img
+            return G(zs_dev, img_size=res, nerf_noise=0.0, **kw)
 
     def step_e2e():
         with torch.no_grad():
@@ -287,11 +303,13 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
         ops.PROFILE = {} if profile else None
+        torch.manual_seed(DRAW_SEED + rank)    # the pre-warm runs for a time, not a count: reseed so every run draws alike
         l0 = lib.c3d_launch_count()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        out = None
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
@@ -302,16 +320,19 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             dist.barrier()
             ms = t.item()
-        return ms, launches, prof
+        return ms, launches, prof, out
 
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms, launches, prof = timed(step_resident, args.steps, args.warmup, profile=True)
-    ms_e2e, _, _ = timed(step_e2e, args.steps, max(1, args.warmup // 2))
+    ms, launches, prof, last = timed(step_resident, args.steps, args.warmup, profile=True)
+    ms_e2e, _, _, _ = timed(step_e2e, args.steps, max(1, args.warmup // 2))
     if sampler:
         sampler.stop_flag = True
         sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"img": last[0], "pitch_yaw": last[1]})
+    del last
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()

@@ -1,5 +1,6 @@
 """Shared helpers for the parity tests (golden loading, oracle replay, error metrics)."""
 import ast
+import json
 import os
 
 import numpy as np
@@ -33,6 +34,51 @@ def oracle_replay(name, dtype=torch.float32):
                                          nerf_noise=meta["nerf_noise"], return_aux_img=True,
                                          return_all=True, **kw)
     return img, py, r, ref
+
+
+def digest(t):
+    """Bit-exact fingerprint of a tensor / array (dtype, shape and bytes): torch.equal against a stored value."""
+    import hashlib
+    a = t.detach().cpu().contiguous().numpy() if isinstance(t, torch.Tensor) else np.ascontiguousarray(t)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()[:16]
+
+
+def digests(sd):
+    return {k: digest(v) for k, v in sd.items()}
+
+
+def digest_all(sd):
+    """One digest of a whole state_dict: its keys in order and every tensor's digest."""
+    return digest(np.array(json.dumps(list(digests(sd).items()))))
+
+
+def sample(t, k=2048, seed=0):
+    """A fixed, seeded sample of k elements of t (all of them when t is smaller): the stored part of a large output."""
+    flat = t.detach().reshape(-1)
+    if flat.numel() <= k:
+        return flat.clone()
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(seed))[:k].sort().values
+    return flat[idx]
+
+
+N_PROJ = 32
+# ||P d|| / sqrt(N_PROJ) lies within [0.47, 1.64] x ||d|| for a fixed d, but with probability 1e-6 at either end
+# (chi-square with N_PROJ degrees of freedom): the slack of an L2 bound checked through projections()
+JL_SLACK = 1.64
+
+
+def projections(t, seed=0, m=N_PROJ):
+    """m seeded Gaussian projections <r_i, t> of the whole of t (accumulated in float64).  ||P a - P b|| / sqrt(m) estimates
+    ||a - b|| (Johnson-Lindenstrauss), so the stored projections of a reference tensor too large to store check an L2 bound
+    over all of its elements."""
+    flat = t.detach().reshape(-1).double()
+    g = torch.Generator().manual_seed(seed)
+    return torch.stack([torch.randn(flat.numel(), generator=g).double() @ flat for _ in range(m)])
+
+
+def projected_l2(t, proj_ref, seed=0):
+    """the estimate of ||t - ref|| from ref's stored projections (same seed)"""
+    return ((projections(t, seed, proj_ref.numel()) - proj_ref.double()).norm() / proj_ref.numel() ** 0.5).item()
 
 
 def rel_err(a, b):

@@ -11,7 +11,6 @@ for p in (ROOT, os.path.join(ROOT, "tools")):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference checkout at /root/reference")
 
 
 # C3D_GPU_TESTS_ON_EMU=1: dry-run the -m gpu tests WITHOUT a GPU -- module-level DEV becomes "cpu" and every test body runs

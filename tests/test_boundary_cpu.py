@@ -5,15 +5,16 @@ import json
 import os
 import re
 
+import numpy as np
 import pytest
 import torch
 
 import ref_shim
 from oracle import cips3d_oracle as O
-from _util import GOLDEN
+from _util import GOLDEN, JL_SLACK, digest, projected_l2, sample
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-needs_ref = pytest.mark.skipif(not ref_shim.reference_available(), reason="no /root/reference")
+PINS = np.load(os.path.join(GOLDEN, "reference_pins.npz"))     # the reference's side of the parity tests
 
 
 @pytest.fixture(scope="module")
@@ -52,20 +53,21 @@ def test_discriminator_state_dict_contract(pkg):
     assert sum(p.numel() for p in D.parameters()) == 37518914          # BASELINE.md section 2
 
 
-@needs_ref
 def test_constructor_init_matches_reference_bitwise(pkg):
-    torch.manual_seed(1234)
-    ref = ref_shim.build_reference_generator().state_dict()
+    """Both constructors initialise like the reference's under the same seed: digests of the reference's state_dicts
+    (tests/golden/reference_pins.npz, tools/make_golden_reference_pins.py)."""
     torch.manual_seed(1234)
     mine = pkg.GeneratorNerfINR(**O.G_CFG, device="cpu").state_dict()
+    ref = json.loads(str(PINS["G_init_1234"]))
+    assert list(ref) == list(mine)
     for k in ref:
-        assert torch.equal(ref[k], mine[k]), k
-    torch.manual_seed(77)
-    refd = ref_shim.build_reference_discriminator().state_dict()
+        assert digest(mine[k]) == ref[k], k
     torch.manual_seed(77)
     myd = pkg.Discriminator_MultiScale_Aux(**ref_shim.D_CFG).state_dict()
+    refd = json.loads(str(PINS["D_init_77"]))
+    assert list(refd) == list(myd)
     for k in refd:
-        assert torch.equal(refd[k], myd[k]), k
+        assert digest(myd[k]) == refd[k], k
 
 
 def test_library_exports_every_declared_symbol(pkg):
@@ -111,35 +113,31 @@ def test_get_zs_and_draw_order(pkg):
     assert len(parts) == 2 and parts[0]["z_nerf"].shape == (2, 256)
 
 
-@needs_ref
 @pytest.mark.parametrize("mode", ["uniform", "normal", "gaussian", "truncated_gaussian", "spherical_uniform", "mean", "hybrid"])
 def test_camera_sampling_matches_reference(pkg, mode):
     import random
-    ref_shim.install()
-    from exp.comm import comm_utils as ref_cu
     kw = dict(bs=5, r=1, horizontal_stddev=0.3, vertical_stddev=0.155, horizontal_mean=1.2, vertical_mean=1.7, mode=mode)
-    torch.manual_seed(9); random.seed(4)
-    a = ref_cu.sample_camera_positions(device="cpu", **kw)
+    a = [torch.from_numpy(PINS[k]) for k in sorted(k for k in PINS.files if re.fullmatch(f"cam_{mode}_[0-9]+", k))]
     torch.manual_seed(9); random.seed(4)
     b = pkg.comm_utils.sample_camera_positions("cpu", **kw)
+    assert len(a) == len(b)
     for x, y in zip(a, b):
-        assert torch.allclose(x, y, atol=1e-6), mode
-    m_ref = ref_cu.create_cam2world_matrix(ref_cu.normalize_vecs(-a[0]), a[0], device="cpu")
+        assert x.shape == y.shape and torch.allclose(x, y, atol=1e-6), mode
+    m_ref = torch.from_numpy(PINS[f"cam_{mode}_cam2world"])
     m = pkg.comm_utils.create_cam2world_matrix(-b[0], b[0], device="cpu")
     assert torch.allclose(m_ref, m, atol=1e-6)
 
 
-@needs_ref
 def test_diffaugment_matches_reference(pkg):
-    ref_shim.install()
-    from exp.cips3d.models.diffaug import DiffAugment as ref_aug
-    x = torch.randn(6, 3, 32, 32)
+    """The reference's DiffAugment output on the same input and seeds.  Stored: a fixed sample of each output's elements,
+    checked at allclose's per-element bound, and Gaussian projections of the whole output, checked against that bound in L2."""
+    x = torch.randn(6, 3, 32, 32, generator=torch.Generator().manual_seed(31))
     for seed in range(5):
         torch.manual_seed(seed)
-        a = ref_aug(x, policy="color,translation,cutout")
-        torch.manual_seed(seed)
         b = pkg.DiffAugment(x, policy="color,translation,cutout")
-        assert torch.allclose(a, b, atol=1e-6), seed
+        assert list(b.shape) == PINS[f"diffaug{seed}_shape"].tolist()
+        assert torch.allclose(torch.from_numpy(PINS[f"diffaug{seed}_sample"]), sample(b, 1024, seed=seed), atol=1e-6), seed
+        assert projected_l2(b, torch.from_numpy(PINS[f"diffaug{seed}_proj"]), seed=seed) < JL_SLACK * float(PINS[f"diffaug{seed}_tol_l2"]), seed
 
 
 def test_scatter_points_roundtrip(pkg):

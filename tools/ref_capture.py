@@ -1,5 +1,6 @@
 """Run the real reference generator while recording every torch.rand/randn draw
-(TEST INFRASTRUCTURE; needs /root/reference)."""
+(TEST INFRASTRUCTURE: the golden generators record the reference's draws with it; the tests
+replay them through draws_from_log)."""
 import contextlib
 import torch
 

@@ -1,7 +1,8 @@
-"""Import shim that lets the UNMODIFIED reference (/root/reference) run on CPU.
+"""Import shim that lets the UNMODIFIED reference (a checkout at $CIPS3D_REFERENCE) run on CPU.
 
-TEST INFRASTRUCTURE ONLY.  Used by tools/make_golden.py and by the (skipped when
-/root/reference is absent) oracle-pinning tests.  Never imported by the product.
+TEST INFRASTRUCTURE ONLY.  Used by the tools/make_golden*.py scripts, which store what the
+reference computes under tests/golden for the parity tests, and by bench.py's reference legs;
+the tests take only its configuration constants.  Never imported by the product.
 
 The reference depends on the author's un-vendored `tl2` package (README.md:62, no
 version pin) plus `easydict` and `streamlit`; none of them contributes arithmetic to
